@@ -5,12 +5,14 @@
     python bench.py --impl reference [--gpus N] ...                 # the reference's CPU algorithm (Python port)
     torchrun --nproc-per-node N ... bench.py --gpus N ...           # one rank per GPU, images sharded (weak scaling)
     python bench.py --config {p30,p10,f64,512}                      # the other single-GPU configurations (default p30)
+    python bench.py --dump-outputs DIR                              # also write the last timed step's person lists to DIR
 
 One pass = the hot path (peaks -> candidate scoring -> greedy matching -> person assembly + wire records, the window
 /root/reference/evaluate.py:507-513 times plus the format_results payload) over one batch of images resident in HBM.
-A "step" is `passes_per_step` passes (so that K steps time >= 100 ms of device work; every pass streams the whole
-input batch, which is larger than L2, from HBM).  At N > 1 every rank's assemble kernel stores its wire records
-straight into rank 0's sink buffer over NVLink (sharding.PeerWireSink): the gather is part of every pass.
+A "step" is `passes_per_step` passes, as many as make one step >= STEP_MS of device work, and `--steps K` times K
+steps (every pass streams the whole input batch, which is larger than L2, from HBM).  At N > 1 every rank's assemble
+kernel stores its wire records straight into rank 0's sink buffer over NVLink (sharding.PeerWireSink): the gather is
+part of every pass.
 One JSON line is printed by rank 0:
 
   value      whole-job images/s with the maps already resident in HBM, CUDA-event timed, max over ranks
@@ -30,6 +32,7 @@ import os
 import statistics
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 import zlib
@@ -40,6 +43,7 @@ sys.path.insert(0, ROOT)
 import numpy as np  # noqa: E402
 
 UNIT = "images/s"
+STEP_MS = 5.0  # device time one step covers at least (the default 20 steps: >= 100 ms)
 BASE_SEED = 20260921
 CAP_ROWS = 64  # person-row capacity of the handles and of a wire record (<= 40 persons/image here; overflow trips the status assert)
 
@@ -74,7 +78,7 @@ def parse_args():
     ap.add_argument("--config", choices=sorted(CONFIGS), default="p30")
     ap.add_argument("--batch", type=int, default=0, help="images per GPU per pass (0 = the configuration's)")
     ap.add_argument("--persons", type=int, default=0, help="0 = the configuration's")
-    ap.add_argument("--passes", type=int, default=0, help="passes per step (0 = as many as make K steps >= 100 ms)")
+    ap.add_argument("--passes", type=int, default=0, help="passes per step (0 = as many as make a step >= STEP_MS)")
     ap.add_argument("--e2e-steps", type=int, default=0, help="0 = min(steps, 10)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-peer", action="store_true", help="N > 1: packed NCCL gather instead of NVLink peer stores")
@@ -82,11 +86,17 @@ def parse_args():
     ap.add_argument("--unfused", action="store_true", help="limb_match and assemble as two kernels instead of the fused match_assemble")
     ap.add_argument("--unmodified", action="store_true",
                     help="--impl reference only, build container only: time the UNMODIFIED reference functions (oracle/ref_loader)")
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="write the person lists the last timed step computed to DIR/<name>.npy (float64)")
     args = ap.parse_args()
+    if args.steps < 1:
+        raise SystemExit("--steps must be at least 1")
     cfg = CONFIGS[args.config]
     args.batch = args.batch or cfg["batch"]
     args.persons = args.persons or cfg["persons"]
     args.H, args.W, args.paf = cfg["H"], cfg["W"], cfg["paf"]
+    if args.impl == "reference" and args.dump_outputs:
+        raise SystemExit("--dump-outputs writes what the CUDA path computed: it does not apply to --impl reference")
     if args.impl == "reference" and "scales" in cfg:
         raise SystemExit("the reference arm times the grouping window (evaluate.py:507-513): use --config p30 / p10 / f64")
     return args
@@ -122,10 +132,12 @@ def make_shard(args, rank):
 
 
 def build_once():
-    """Every rank calls this; a file lock makes one of them compile while the others wait for the finished library."""
+    """Every rank calls this; a file lock makes one of them compile while the others wait for the finished library.
+    The lock lives in the temporary directory: the source tree may be read-only."""
     import __graft_entry__ as ge
 
-    with open(os.path.join(ROOT, ".build.lock"), "w") as fh:
+    lock = os.path.join(tempfile.gettempdir(), f"spgroup-build-{zlib.crc32(ROOT.encode()):08x}.lock")
+    with open(lock, "w") as fh:
         fcntl.flock(fh, fcntl.LOCK_EX)
         try:
             ge.build()
@@ -145,6 +157,28 @@ def host_cpu_budget():
         pass
     usable = min(affinity, quota) if quota else affinity
     return {"os_cpu_count": os.cpu_count(), "affinity": affinity, "cgroup_quota_cpus": quota, "usable": usable}
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(dirname, views, B):
+    """--dump-outputs: what a caller of the timed path receives -- person counts, keypoint coordinates, person scores and
+    status flags -- as float64 ``DIR/<name>.npy``.  Rows at or beyond an image's person count are never written by the
+    kernels and hold whatever an earlier pass left there, so they are stored as zeros.  Larger than DUMP_LIMIT_BYTES in
+    all, a fixed seeded sample of the images is written, their indices in ``image_index.npy``."""
+    out = {k: views[k][:B].cpu().numpy().astype(np.float64) for k in ("n_persons", "people_xy", "people_score", "status")}
+    live = np.arange(out["people_score"].shape[1])[None, :] < out["n_persons"][:, None]
+    out["people_xy"][~live] = 0.0
+    out["people_score"][~live] = 0.0
+    per_image = sum(v[0].nbytes for v in out.values()) + 8  # + its entry in image_index
+    if B * per_image > DUMP_LIMIT_BYTES:
+        idx = np.sort(np.random.default_rng(BASE_SEED).choice(B, DUMP_LIMIT_BYTES // per_image, replace=False))
+        out = {k: v[idx] for k, v in out.items()}
+        out["image_index"] = idx.astype(np.float64)
+    os.makedirs(dirname, exist_ok=True)
+    for k, v in out.items():
+        np.save(os.path.join(dirname, k + ".npy"), v)
 
 
 # ------------------------------------------------------------------------------------------------------
@@ -367,7 +401,7 @@ def run_ours(args, rank, world, local_rank):
         one_pass()
     join_consumer()
     barrier()
-    # ---- passes per step: enough that K steps cover >= 100 ms of device time (same number on every rank)
+    # ---- passes per step: enough that a step covers >= STEP_MS of device time (same number on every rank)
     passes = args.passes
     if passes <= 0:
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
@@ -380,7 +414,7 @@ def run_ours(args, rank, world, local_rank):
         t = torch.tensor([e0.elapsed_time(e1) / 4], dtype=torch.float64, device=dev)
         if world > 1:
             dist.all_reduce(t, op=dist.ReduceOp.MIN)
-        passes = max(1, min(64, math.ceil(100.0 / (args.steps * float(t.item())))))
+        passes = max(1, min(64, math.ceil(STEP_MS / float(t.item()))))
     for _ in range(max(args.warmup, 3)):
         for _ in range(passes):
             one_pass()
@@ -401,6 +435,8 @@ def run_ours(args, rank, world, local_rank):
     torch.cuda.synchronize()
     w1 = time.time()
     launches = g.launch_count - l0
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, views, B)
     barrier()
     elapsed_ms = ev_start.elapsed_time(ev_end)
     used = [e for k, e in enumerate(evs) if passes > 1 or k % 5 == 0]
@@ -678,7 +714,7 @@ def run_pipeline(args, local_rank):
         one_pass()
     e1.record(stream)
     torch.cuda.synchronize()
-    passes = args.passes or max(1, min(64, math.ceil(100.0 / (args.steps * e0.elapsed_time(e1) / 4))))
+    passes = args.passes or max(1, min(64, math.ceil(STEP_MS / (e0.elapsed_time(e1) / 4))))
     for _ in range(max(args.warmup, 3) * passes):
         one_pass()
     torch.cuda.synchronize()
@@ -700,6 +736,8 @@ def run_pipeline(args, local_rank):
     l0 = g.launch_count
     elapsed_ms, stage_ms = timed(0)          # value: post-network stage + grouping
     launches = g.launch_count - l0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, views, B)
     group_ms, _ = timed(n_pre)               # the grouping stages alone on the resident maps
     n_pass = args.steps * passes
     value = B * n_pass / (elapsed_ms / 1e3)

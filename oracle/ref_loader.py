@@ -2,8 +2,8 @@
 
 TEST INFRASTRUCTURE ONLY.  This module works only where ``/root/reference``
 exists (the build container); it never travels to the GPU box.  It is used by
-``tests/golden/make_golden.py`` (fixture generation) and by the optional
-``tests/test_oracle_vs_reference.py`` (skipped when the reference is absent).
+``tests/golden/make_golden.py`` and ``tests/golden/make_reference_outputs.py``
+(fixture generation).
 
 ``import evaluate`` cannot work here (pycocotools / matplotlib / configobj /
 apex are missing and the module body parses ``sys.argv`` and pins

@@ -53,6 +53,26 @@ def unflatten(d) -> tuple:
     return all_peaks, connection_all, [int(v) for v in d["special_k"]], np.array(d["subset"]), np.array(cand)
 
 
+def stack(flats) -> dict:
+    """Several ``flatten`` dicts as one: each field concatenated along axis 0, its per-dict lengths in ``<field>_len``."""
+    out = {}
+    for k in flats[0]:
+        out[k] = np.concatenate([f[k] for f in flats])
+        out[k + "_len"] = np.array([len(f[k]) for f in flats], np.int64)
+    return out
+
+
+def unstack(d, j: int) -> dict:
+    """The ``j``-th ``flatten`` dict of a ``stack`` result."""
+    out = {}
+    for k in d:
+        if k + "_len" in d:
+            n = d[k + "_len"]
+            a = int(n[:j].sum())
+            out[k] = d[k][a:a + int(n[j])]
+    return out
+
+
 def save_case(path, heat, paf, limbs, image_extent, params, structs, meta=None) -> None:
     np.savez_compressed(path, heat=heat, paf=paf, limbs=np.asarray(limbs, np.int32), image_extent=np.int64(image_extent),
                         params=np.array(json.dumps(params)), meta=np.array(json.dumps(meta or {})), **flatten(structs))

@@ -404,7 +404,7 @@ def test_random_parameters_and_dirt_against_the_checker(env):
     """40 seeded draws of (hyper-parameters x dirty-input knobs x map shape): every combination the CUDA path can be
     configured with must reproduce the checker, floats included.  Covers offset_radius 0..4, mid_num 1..40 (per-m
     tables), connect_ration / thresholds that move maxfail, remove_recon, len_rate / connection_tole rejects."""
-    from test_oracle_vs_reference import fuzz_cases  # the same draws are checked against the live reference on CPU
+    from test_oracle_vs_reference import fuzz_cases  # the same draws are checked against the reference's outputs on CPU
 
     for trial, heat, paf, extent, params, cap in fuzz_cases(40):
         o = env.so.group_batch(heat, paf, env.skeleton.LIMBS, extent, params)

@@ -1,18 +1,18 @@
 """CPU: the inference IMHN (improved_body_parts_b200/imhn.py, SURVEY.md §8 f-3) against the reference's own module.
 
-Where /root/reference is present (build container) the reference's ``NetworkEval`` (models/posenet.py:175-193) is
-instantiated, its state dict is loaded into ours with ``strict=True`` (same parameter names and shapes: reference
-checkpoints load, evaluate.py:629-630) and the outputs are compared: all ``nstack x 5`` maps of ``forward_all`` and the
-single tensor ``forward`` returns (= ``output_tuple[-1][0]``, evaluate.py:126).  Elsewhere only the self-consistency
-checks run (BatchNorm folding, pruned vs full forward)."""
+The reference's ``NetworkEval`` (models/posenet.py:175-193) state dict names and shapes, and its outputs for fixed
+deterministic weights, are stored in tests/golden/reference/imhn.npz (tests/golden/make_reference_outputs.py).  The
+same weights are loaded into ours with ``strict=True`` (same parameter names and shapes: reference checkpoints load,
+evaluate.py:629-630) and the outputs are compared: all ``nstack x 5`` maps of ``forward_all`` and the single tensor
+``forward`` returns (= ``output_tuple[-1][0]``, evaluate.py:126).  The self-consistency checks (BatchNorm folding,
+pruned vs full forward) need no stored data."""
+import math
 import os
-import sys
 
-import pytest
+import numpy as np
 import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = os.environ.get("SPG_REFERENCE_ROOT", "/root/reference")
 
 
 def _small(nstack=2):
@@ -48,41 +48,63 @@ def test_pruned_forward_is_the_last_stacks_finest_map_and_bn_folding_is_exact_en
     assert torch.allclose(folded, one, rtol=1e-4, atol=1e-5 * float(one.abs().max()))
 
 
-@pytest.mark.skipif(not os.path.isfile(os.path.join(REF, "models", "posenet.py")), reason="needs /root/reference")
+def seeded_state(entries, seed=1):
+    """Deterministic values for a state dict given as ``(name, shape)`` pairs: weight matrices and kernels uniform in
+    +-1/sqrt(fan_in) (PyTorch's default bound), BatchNorm scales and statistics away from the identity, small biases."""
+    g = torch.Generator().manual_seed(seed)
+    out = {}
+    for name, shape in entries:
+        leaf = name.rsplit(".", 1)[-1]
+        if leaf == "num_batches_tracked":
+            out[name] = torch.zeros(shape, dtype=torch.long)
+            continue
+        if leaf == "running_mean":
+            lo, hi = -0.2, 0.2
+        elif leaf == "running_var" or (leaf == "weight" and len(shape) == 1):
+            lo, hi = 0.5, 1.5
+        elif len(shape) > 1:
+            hi = math.prod(shape[1:]) ** -0.5
+            lo = -hi
+        else:
+            lo, hi = -0.1, 0.1
+        out[name] = torch.rand(shape, generator=g) * (hi - lo) + lo
+    return out
+
+
+def imhn_input():
+    return torch.rand(2, 64, 64, 3, generator=torch.Generator().manual_seed(2))
+
+
+def map_sample(t, n=256):
+    """A fixed, evenly strided sample of at most about ``n`` values of a map, as float32."""
+    flat = t.detach().reshape(-1)
+    return flat[::max(1, flat.numel() // n)].numpy().astype(np.float32)
+
+
 def test_reference_state_dict_loads_strictly_and_outputs_agree():
-    import contextlib
-    import io
-    import types
+    """The reference's ``NetworkEval`` state dict (names and shapes) loads with ``strict=True`` and, for the same
+    deterministic weights, every map of ``forward_all`` and the tensor ``forward`` returns agree with the reference's
+    outputs (tests/golden/reference/imhn.npz: a fixed sample of each map and the map's largest magnitude)."""
+    import json
 
     from improved_body_parts_b200.imhn import IMHN
-    sys.path.insert(0, REF)
-    try:
-        with contextlib.redirect_stdout(io.StringIO()):
-            from models.posenet import NetworkEval  # the reference's module, unmodified
-    finally:
-        sys.path.remove(REF)
-    opt = types.SimpleNamespace(nstack=4, hourglass_inp_dim=256, increase=128)
-    cfg = types.SimpleNamespace(num_layers=50)
-    torch.manual_seed(1)
-    ref = NetworkEval(opt, cfg, bn=True).eval()
-    with torch.no_grad():
-        for mod in ref.modules():
-            if isinstance(mod, torch.nn.BatchNorm2d):
-                mod.running_mean.uniform_(-0.2, 0.2)
-                mod.running_var.uniform_(0.5, 1.5)
+    with np.load(os.path.join(ROOT, "tests", "golden", "reference", "imhn.npz"), allow_pickle=False) as z:
+        ref = {k: z[k] for k in z.files}
+    entries = json.loads(str(ref["state"]))
     ours = IMHN(nstack=4)
-    missing = ours.load_state_dict(ref.state_dict(), strict=True)  # same names, same shapes
+    missing = ours.load_state_dict(seeded_state(entries), strict=True)  # same names, same shapes
     assert not missing.missing_keys and not missing.unexpected_keys
-    assert sum(p.numel() for p in ours.parameters()) == sum(p.numel() for p in ref.parameters()) > 100e6
-    x = torch.rand(2, 64, 64, 3)
+    assert sum(p.numel() for p in ours.parameters()) == sum(math.prod(s) for k, s in entries if "running" not in k
+                                                            and "num_batches" not in k) > 100e6
+    x = imhn_input()
     with torch.no_grad():
-        want = ref(x)
         got = ours.forward_all(x)
         worst = 0.0
         for i in range(4):
             for j in range(5):
-                scale = float(want[i][j].abs().max())
-                worst = max(worst, float((got[i][j] - want[i][j]).abs().max()) / scale)
+                scale = float(ref[f"s{i}_{j}_absmax"])
+                assert scale > 1e-3
+                worst = max(worst, float(np.abs(map_sample(got[i][j]) - ref[f"s{i}_{j}_sample"]).max()) / scale)
         # same float32 network; only the association of a few sums differs (x + (a + b) vs (x + a) + b, mean vs avg-pool)
         assert worst < 2e-5, worst
-        assert float((ours(x) - want[-1][0]).abs().max()) / float(want[-1][0].abs().max()) < 2e-5
+        assert float(np.abs(map_sample(ours(x)) - ref["s3_0_sample"]).max()) / float(ref["s3_0_absmax"]) < 2e-5

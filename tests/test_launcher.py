@@ -1,7 +1,8 @@
-"""CPU, build container only (needs /root/reference): the launcher that runs ``evaluate.py`` unchanged
-(tools/run_evaluate_b200.py) against the REAL module -- import with stubbed third-party modules, CUDA_VISIBLE_DEVICES
-restored after the module pins it (evaluate.py:28), the three call-site names rebound (:509-511), ``limbSeq`` picked
-up (:54), ``params`` read from the reference's own utils/config, and ``format_results`` replaceable."""
+"""CPU: the launcher that runs ``evaluate.py`` unchanged (tools/run_evaluate_b200.py) against the REAL module, where a
+reference checkout is present -- import with stubbed third-party modules, CUDA_VISIBLE_DEVICES restored after the
+module pins it (evaluate.py:28), the three call-site names rebound (:509-511), ``limbSeq`` picked up (:54), ``params``
+read from the reference's own utils/config, and ``format_results`` replaceable -- and the INI reader against what it
+made of that utils/config."""
 import importlib.util
 import os
 import subprocess
@@ -12,7 +13,6 @@ import pytest
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 REF = os.environ.get("SPG_REFERENCE_ROOT", "/root/reference")
 
-pytestmark = pytest.mark.skipif(not os.path.isfile(os.path.join(REF, "evaluate.py")), reason="needs /root/reference")
 
 _CHILD = r'''
 import json, os, sys
@@ -39,6 +39,7 @@ print("RESULT " + json.dumps(out))
 '''
 
 
+@pytest.mark.skipif(not os.path.isfile(os.path.join(REF, "evaluate.py")), reason="needs the reference checkout's evaluate.py")
 def test_launcher_imports_the_real_evaluate_and_rebinds_it():
     import json
     r = subprocess.run([sys.executable, "-c", _CHILD.format(root=ROOT, ref=REF)], capture_output=True, text=True, timeout=300)
@@ -55,9 +56,12 @@ def test_launcher_imports_the_real_evaluate_and_rebinds_it():
 
 
 def test_ini_reader_agrees_with_the_reference_config_file():
+    import json
     sys.path.insert(0, ROOT)
     from improved_body_parts_b200 import skeleton
-    param, model = skeleton.read_reference_ini(os.path.join(REF, "utils", "config"))
+    # what the reader made of the reference's own utils/config (tests/golden/make_reference_outputs.py)
+    stored = json.load(open(os.path.join(ROOT, "tests", "golden", "reference", "utils_config.json")))
+    param, model = stored["param"], stored["model"]
     fixture = skeleton.read_reference_ini(os.path.join(ROOT, "tests", "golden", "reference_utils_config.ini"))
     assert param == fixture[0]
     assert {k: model[k] for k in ("boxsize", "padValue", "stride", "max_downsample")} == \

@@ -1,11 +1,12 @@
 """CPU: wire records (improved_body_parts_b200/wire.py) -- the ``format_results`` payload (evaluate.py:563-582).
 
 The record layout is checked against the C header's formula, pack/unpack round-trips the reference's Python
-structures (integer ``(0, 0)`` placeholders included), and -- where /root/reference is present -- the JSON written by
-``wire.format_results`` is compared byte for byte with the file the reference's own ``format_results`` writes for the
-people lists its own ``process()`` tail builds on the goldens."""
+structures (integer ``(0, 0)`` placeholders included), and the JSON written by ``wire.format_results`` is compared
+byte for byte with the file the reference's own ``format_results`` wrote for the people lists its own ``process()``
+tail builds on the goldens (tests/golden/reference/format_results.json, tests/golden/make_reference_outputs.py)."""
 import json
 import os
+from pathlib import Path
 
 import numpy as np
 import pytest
@@ -78,13 +79,9 @@ def test_pack_unpack_round_trip_keeps_placeholders_and_bits():
 
 def test_format_results_writes_the_reference_file(tmp_path):
     from improved_body_parts_b200 import wire
-    from oracle import ref_loader
-    if not ref_loader.reference_available():
-        pytest.skip("needs /root/reference (build container)")
     people = _golden_people()
-    ref_fn = ref_loader.reference_function("format_results")
-    a, b, c = tmp_path / "ref.json", tmp_path / "ours.json", tmp_path / "wire.json"
-    ref_fn(people, str(a))
+    a = Path(__file__).parent / "golden" / "reference" / "format_results.json"  # what the reference's format_results wrote
+    b, c = tmp_path / "ours.json", tmp_path / "wire.json"
     wire.format_results(people, str(b))
     assert a.read_bytes() == b.read_bytes()
     # ... and through the binary records (what the GPU emits): same bytes again
