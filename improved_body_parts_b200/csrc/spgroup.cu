@@ -9,6 +9,7 @@
 #include <cuda_runtime.h>
 
 #include <algorithm>
+#include <cmath>
 #include <cstdarg>
 #include <cstdio>
 #include <cstdlib>
@@ -27,6 +28,7 @@
 #include "nms_peaks_persist.cuh"
 #include "nms_peaks_banded.cuh"
 #include "postnet.cuh"
+#include "postnet_rot.cuh"
 
 using namespace spg;
 
@@ -600,9 +602,13 @@ int64_t spg_launch_count(const spg_handle *h) { return h ? h->launches : 0; }
 const char *spg_stage_kernel(const spg_handle *h, int32_t stage) { return (h && stage >= 0 && stage < 5) ? h->stage_kernel[stage] : ""; }
 
 // ---- post-network stage ------------------------------------------------------------------------
-int spg_postnet(spg_handle *h, const spg_postnet_desc *d, int32_t n, int32_t H, int32_t W, float *heat_out, void *paf_out,
-                int32_t paf_dtype, void *stream) {
-    if (!h) return SPG_E_INVALID;
+namespace {
+
+// Checks shared by spg_postnet and spg_postnet_rotated; allocates the float64 keypoint sums when they outlive a launch
+// and fills the arguments common to every launch of the call.  *done is set when there is nothing to launch (n == 0).
+int postnet_setup(spg_handle *h, const spg_postnet_desc *d, int32_t n, int32_t H, int32_t W, float *heat_out, void *paf_out,
+                  int32_t paf_dtype, bool rotated, PostArgs &a, bool *done) {
+    *done = true;
     if (!d || !d->scales || d->n_scales < 1 || !d->flip_paf_ord || !d->flip_heat_ord) return fail(h, SPG_E_INVALID, "postnet descriptor incomplete");
     if ((!heat_out || !paf_out) && n > 0) return fail(h, SPG_E_INVALID, "heat_out/paf_out is NULL");
     if (paf_dtype != SPG_F32 && paf_dtype != SPG_F64) return fail(h, SPG_E_INVALID, "paf_dtype must be SPG_F32 or SPG_F64");
@@ -615,19 +621,18 @@ int spg_postnet(spg_handle *h, const spg_postnet_desc *d, int32_t n, int32_t H, 
     const Workspace &ws = h->ws;
     if (ws.K + ws.L > kMaxNetChannels) return fail(h, SPG_E_INVALID, "too many channels for postnet");
     DeviceGuard guard(h->device);
-    cudaStream_t st = static_cast<cudaStream_t>(stream);
-    if (d->n_scales > 1 && (d->stride != 4 || d->n_scales > kPostMaxScales)) {  // float64 keypoint sums that outlive a launch
+    // float64 keypoint sums that outlive a launch: rotated items run one launch each
+    if (d->n_scales > 1 && (rotated || d->stride != 4 || d->n_scales > kPostMaxScales)) {
         const size_t need = (size_t)h->cfg.max_batch * ws.K * H * W;
         if (h->heat_acc_elems < need) {
             if (h->heat_acc) cudaFree(h->heat_acc);
-    if (h->done_counter) cudaFree(h->done_counter);
             h->heat_acc = nullptr; h->heat_acc_elems = 0;
             SPG_CUDA(h, cudaMalloc(&h->heat_acc, need * sizeof(double)));
             h->heat_acc_elems = need;
         }
     }
     // validate every scale and fill the common arguments
-    PostArgs a{};
+    a = PostArgs{};
     a.stride = d->stride; a.H = H; a.W = W; a.n_out = ws.K + ws.L; a.K = ws.K;
     for (int c = 0; c < ws.K; c++) {
         if (d->flip_heat_ord[c] < 0 || d->flip_heat_ord[c] >= ws.K) return fail(h, SPG_E_INVALID, "flip_heat_ord[%d] out of range", c);
@@ -649,16 +654,25 @@ int spg_postnet(spg_handle *h, const spg_postnet_desc *d, int32_t n, int32_t H, 
         if (sc.h < 1 || sc.w < 1 || sc.crop_h < 1 || sc.crop_w < 1 || sc.crop_h > sc.h * d->stride || sc.crop_w > sc.w * d->stride)
             return fail(h, SPG_E_INVALID, "scale %d: crop %dx%d does not fit the up-sampled %dx%d output", t, sc.crop_h, sc.crop_w, sc.h * d->stride, sc.w * d->stride);
     }
-    auto scale_of = [&](const spg_postnet_scale &sc) {
-        PostScale s{};
-        s.net = sc.net_out; s.net_is_f16 = sc.dtype == SPG_F16;
-        s.img_stride = sc.image_stride; s.pair_stride = sc.pair_stride; s.chan_stride = sc.chan_stride;
-        s.h = sc.h; s.w = sc.w; s.crop_h = sc.crop_h; s.crop_w = sc.crop_w;
-        // cv2.resize(dsize): inv_scale = dst/src, scale = 1/inv_scale (two roundings, as OpenCV)
-        s.sx2 = 1.0 / ((double)W / (double)sc.crop_w);
-        s.sy2 = 1.0 / ((double)H / (double)sc.crop_h);
-        return s;
-    };
+    *done = false;
+    return SPG_OK;
+}
+
+PostScale postnet_scale_of(const spg_postnet_scale &sc, int H, int W) {
+    PostScale s{};
+    s.net = sc.net_out; s.net_is_f16 = sc.dtype == SPG_F16;
+    s.img_stride = sc.image_stride; s.pair_stride = sc.pair_stride; s.chan_stride = sc.chan_stride;
+    s.h = sc.h; s.w = sc.w; s.crop_h = sc.crop_h; s.crop_w = sc.crop_w;
+    // cv2.resize(dsize): inv_scale = dst/src, scale = 1/inv_scale (two roundings, as OpenCV)
+    s.sx2 = 1.0 / ((double)W / (double)sc.crop_w);
+    s.sy2 = 1.0 / ((double)H / (double)sc.crop_h);
+    return s;
+}
+
+// The items [t_begin, t_end) of the loop (angle 0) with the stride-4 or the generic kernels; a.n_scales is the length of
+// the whole loop, so sums that continue from earlier items, or into later ones, go through memory.
+int postnet_launch_items(spg_handle *h, PostArgs &a, const spg_postnet_desc *d, int t_begin, int t_end, int32_t n, int32_t H,
+                         int32_t W, cudaStream_t st) {
     // output tile: as large as the shared-memory tiles of the intermediate / source allow
     auto tile_dim = [&](double s2, double s1, int cap1, int cap0, int maxd, double margin) {
         const double c1 = std::min((double)cap1, ((double)cap0 - 7.0) / s1) - margin;  // intermediate span allowed
@@ -667,12 +681,12 @@ int spg_postnet(spg_handle *h, const spg_postnet_desc *d, int32_t n, int32_t H, 
     const bool fast = d->stride == 4;  // the reference's model: four-phase kernel; other strides: table-driven generic kernel
     if (fast) {
         // the scale loop runs INSIDE the kernel (groups of kPostMaxScales): one tile geometry for all fused scales
-        for (int t0 = 0; t0 < d->n_scales; t0 += kPostMaxScales) {
-            a.n_fused = std::min(kPostMaxScales, d->n_scales - t0);
+        for (int t0 = t_begin; t0 < t_end; t0 += kPostMaxScales) {
+            a.n_fused = std::min(kPostMaxScales, t_end - t0);
             a.scale_index = t0;
             a.tile_w = kPostTW; a.tile_h = kPostTH;
             for (int t = 0; t < a.n_fused; t++) {
-                a.sc[t] = scale_of(d->scales[t0 + t]);
+                a.sc[t] = postnet_scale_of(d->scales[t0 + t], H, W);
                 a.tile_w = std::min(a.tile_w, tile_dim(a.sc[t].sx2, a.sx1, kPostF_C1, kPostF_CS, kPostTW, 13.0));
                 a.tile_h = std::min(a.tile_h, tile_dim(a.sc[t].sy2, a.sy1, kPostF_R1, kPostF_RS, kPostTH, 13.0));
             }
@@ -725,8 +739,8 @@ int spg_postnet(spg_handle *h, const spg_postnet_desc *d, int32_t n, int32_t H, 
         }
         return SPG_OK;
     }
-    for (int t = 0; t < d->n_scales; t++) {  // generic kernel: one launch per scale, float64 accumulators in memory
-        const PostScale s = scale_of(d->scales[t]);
+    for (int t = t_begin; t < t_end; t++) {  // generic kernel: one launch per scale, float64 accumulators in memory
+        const PostScale s = postnet_scale_of(d->scales[t], H, W);
         a.net = s.net; a.net_is_f16 = s.net_is_f16; a.img_stride = s.img_stride; a.pair_stride = s.pair_stride; a.chan_stride = s.chan_stride;
         a.h = s.h; a.w = s.w; a.crop_h = s.crop_h; a.crop_w = s.crop_w; a.sx2 = s.sx2; a.sy2 = s.sy2;
         a.scale_index = t;
@@ -741,6 +755,121 @@ int spg_postnet(spg_handle *h, const spg_postnet_desc *d, int32_t n, int32_t H, 
         h->stage_kernel[4] = "postnet_generic_kernel";
         h->launches++;
         SPG_CUDA(h, cudaGetLastError());
+    }
+    return SPG_OK;
+}
+
+// cv2.getRotationMatrix2D((rows / 2, cols / 2), angle, 1) -- the centre is a Point2f, (rows, cols) passed as (x, y) as the
+// reference does (evaluate.py:109-110) -- then the inversion cv2.warpAffine applies without WARP_INVERSE_MAP
+// (imgproc/src/imgwarp.cpp), all in float64: the destination -> source map of the warp.
+void rotation_inverse_map(double angle_deg, int rows, int cols, double m[6]) {
+    const double cx = (double)(float)(rows / 2.0), cy = (double)(float)(cols / 2.0);
+    const double ang = angle_deg * (3.14159265358979323846 / 180);
+    const double alpha = std::cos(ang), beta = std::sin(ang);
+    m[0] = alpha; m[1] = beta; m[2] = (1 - alpha) * cx - beta * cy;
+    m[3] = -beta; m[4] = alpha; m[5] = beta * cx + (1 - alpha) * cy;
+    double D = m[0] * m[4] - m[1] * m[3];
+    D = D != 0 ? 1. / D : 0;
+    const double a11 = m[4] * D, a22 = m[0] * D;
+    m[0] = a11; m[1] *= -D;
+    m[3] *= -D; m[4] = a22;
+    const double b1 = -m[0] * m[2] - m[1] * m[5];
+    const double b2 = -m[3] * m[2] - m[4] * m[5];
+    m[2] = b1; m[5] = b2;
+}
+
+// Item t of the loop with a non-zero angle: one postnet_rot_kernel launch.
+int postnet_launch_rotated(spg_handle *h, PostArgs &a, const spg_postnet_desc *d, int t, double angle_deg, int32_t n, int32_t H,
+                           int32_t W, cudaStream_t st) {
+    const PostScale s = postnet_scale_of(d->scales[t], H, W);
+    a.net = s.net; a.net_is_f16 = s.net_is_f16; a.img_stride = s.img_stride; a.pair_stride = s.pair_stride; a.chan_stride = s.chan_stride;
+    a.h = s.h; a.w = s.w; a.crop_h = s.crop_h; a.crop_w = s.crop_w; a.sx2 = s.sx2; a.sy2 = s.sy2;
+    a.scale_index = t;
+    PostRotArgs r{};
+    r.Hp = s.h * a.stride; r.Wp = s.w * a.stride;
+    rotation_inverse_map(-angle_deg, r.Hp, r.Wp, r.m);  // rotate_matrix_reverse (evaluate.py:110)
+    // Tile: the largest of a ladder whose shared-memory tiles fit 64 KB (three CTAs per SM).  Capacities are upper bounds
+    // of the spans the kernel finds: footprint = taps of the second resize (span (tile - 1) * ratio + 4, +1 for float
+    // rounding); box = the footprint's rotated extent (|m0| fw + |m1| fh for x) + 2 for the floors of the fixed-point
+    // taps and the second bilinear tap, +1 spare; source = taps of the x stride resize ((box - 1) / stride + 5, +1).
+    const bool identity = s.crop_h == H && s.crop_w == W;
+    static const int ladder[][2] = {{64, 32}, {32, 32}, {32, 16}, {16, 16}, {16, 8}, {8, 8}, {4, 4}, {2, 2}, {1, 1}};
+    size_t smem = 0;
+    bool fits = false;
+    for (const auto &tl : ladder) {
+        const int tw = std::min(tl[0], W), th = std::min(tl[1], H);
+        const int fw = identity ? tw : std::min(s.crop_w, (int)std::ceil((tw - 1) * s.sx2) + 6);
+        const int fh = identity ? th : std::min(s.crop_h, (int)std::ceil((th - 1) * s.sy2) + 6);
+        const int bw = std::min(r.Wp, (int)std::ceil(std::fabs(r.m[0]) * (fw - 1) + std::fabs(r.m[1]) * (fh - 1)) + 4);
+        const int bh = std::min(r.Hp, (int)std::ceil(std::fabs(r.m[3]) * (fw - 1) + std::fabs(r.m[4]) * (fh - 1)) + 4);
+        const int cs = std::min(s.w, (int)std::ceil((bw - 1) / (double)a.stride) + 6);
+        const int rs = std::min(s.h, (int)std::ceil((bh - 1) / (double)a.stride) + 6);
+        a.tile_w = tw; a.tile_h = th;
+        r.cap_fw = fw; r.cap_fh = fh; r.cap_bw = bw; r.cap_bh = bh; r.cap_cs = cs; r.cap_rs = rs;
+        smem = postrot_smem_bytes(tw, th, fw, fh, bw, bh, cs, rs);
+        if (smem <= 64 * 1024) { fits = true; break; }
+    }
+    if (!fits && smem > h->smem_optin)
+        return fail(h, SPG_E_INVALID, "item %d: a %dx%d crop resized to %dx%d needs %zu bytes of shared memory even for a 1x1 tile", t,
+                    s.crop_h, s.crop_w, H, W, smem);
+    a.tiles_x = (W + a.tile_w - 1) / a.tile_w;
+    a.tiles_y = (H + a.tile_h - 1) / a.tile_h;
+    if ((long long)a.tiles_x * a.tiles_y > 0x7fffffffLL || n > 65535) return fail(h, SPG_E_INVALID, "postnet grid too large");
+    // tables once per CTA, then a chunk of channels: as many chunks as leave ~16 CTAs per SM in the grid
+    const long long tiles = (long long)a.tiles_x * a.tiles_y * n;
+    const int n_chunks = (int)std::min<long long>(a.n_out, std::max<long long>(1, ((long long)h->sm_count * 16 + tiles - 1) / tiles));
+    a.chan_chunk = (a.n_out + n_chunks - 1) / n_chunks;
+    r.a = a;
+    dim3 grid((unsigned)(a.tiles_x * a.tiles_y), (unsigned)((a.n_out + a.chan_chunk - 1) / a.chan_chunk), (unsigned)n);
+    SPG_CUDA(h, cudaFuncSetAttribute(postnet_rot_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    postnet_rot_kernel<<<grid, kPostThreads, smem, st>>>(r);
+    h->stage_kernel[4] = "postnet_rot_kernel";
+    h->launches++;
+    SPG_CUDA(h, cudaGetLastError());
+    return SPG_OK;
+}
+
+}  // namespace
+
+int spg_postnet(spg_handle *h, const spg_postnet_desc *d, int32_t n, int32_t H, int32_t W, float *heat_out, void *paf_out,
+                int32_t paf_dtype, void *stream) {
+    if (!h) return SPG_E_INVALID;
+    PostArgs a;
+    bool done;
+    int rc = postnet_setup(h, d, n, H, W, heat_out, paf_out, paf_dtype, false, a, &done);
+    if (rc || done) return rc;
+    DeviceGuard guard(h->device);
+    return postnet_launch_items(h, a, d, 0, d->n_scales, n, H, W, static_cast<cudaStream_t>(stream));
+}
+
+int spg_postnet_rotated(spg_handle *h, const spg_postnet_desc *d, const double *angle_deg, int32_t n, int32_t H, int32_t W,
+                        float *heat_out, void *paf_out, int32_t paf_dtype, void *stream) {
+    if (!h) return SPG_E_INVALID;
+    if (!d || d->n_scales < 1 || !angle_deg) return fail(h, SPG_E_INVALID, "postnet descriptor incomplete or angle_deg is NULL");
+    bool any_rotated = false;
+    for (int t = 0; t < d->n_scales; t++) {
+        if (!std::isfinite(angle_deg[t])) return fail(h, SPG_E_INVALID, "angle_deg[%d] is not finite", t);
+        any_rotated = any_rotated || angle_deg[t] != 0.0;
+    }
+    if (!any_rotated) return spg_postnet(h, d, n, H, W, heat_out, paf_out, paf_dtype, stream);
+    PostArgs a;
+    bool done;
+    int rc = postnet_setup(h, d, n, H, W, heat_out, paf_out, paf_dtype, true, a, &done);
+    if (rc || done) return rc;
+    DeviceGuard guard(h->device);
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    // items in the order of the loop (scale-major, angle-minor): consecutive angle-0 items go to the existing kernels as
+    // one group, each rotated item is one launch; the float64 sums carry over through memory
+    for (int t = 0; t < d->n_scales;) {
+        if (angle_deg[t] == 0.0) {
+            int t1 = t;
+            while (t1 < d->n_scales && angle_deg[t1] == 0.0) t1++;
+            if ((rc = postnet_launch_items(h, a, d, t, t1, n, H, W, st))) return rc;
+            t = t1;
+        } else {
+            if ((rc = postnet_launch_rotated(h, a, d, t, angle_deg[t], n, H, W, st))) return rc;
+            t++;
+        }
     }
     return SPG_OK;
 }

@@ -18,6 +18,7 @@ There is no CPU path: without the CUDA library / an sm_100 GPU these functions r
 """
 from __future__ import annotations
 
+from itertools import product
 from typing import Dict, List, Optional, Sequence, Tuple
 
 import numpy as np
@@ -117,24 +118,26 @@ def pad_right_down_corner(img: np.ndarray, stride: int, pad_value: int) -> Tuple
 def predict(image, params, model, model_params, heat_layers=None, paf_layers=None, input_image_path=None):
     """evaluate.py:83-166 with everything after the forward pass on the device.
 
-    Same arguments as the reference's ``predict``.  The image is scaled and padded exactly as there (cv2, host), the
-    network runs on the image and its mirror (:116-124), and the flip ensemble, both bicubic resizes, the crop and the
-    float64 average over ``scale_search`` (:126-161) happen in ``spg_postnet`` -- the maps never visit the host.
-    Returns two ``DeviceMaps`` (heatmap, paf) that ``find_peaks`` / ``find_connections`` / ``group`` accept directly.
-    ``rotation_search`` other than ``[0]`` (the reference's default, utils/config:27) is not supported."""
+    Same arguments as the reference's ``predict``.  The image is scaled and padded exactly as there (cv2, host) and,
+    for an item of ``rotation_search`` with a non-zero angle, rotated with ``cv2.warpAffine`` (:108-111, host); the
+    network runs on the image and its mirror (:116-124), and the flip ensemble, both bicubic resizes, the warp back,
+    the crop and the float64 average over ``product(scale_search, rotation_search)`` (:126-161) happen in
+    ``spg_postnet`` / ``spg_postnet_rotated`` -- the maps never visit the host.
+    Returns two ``DeviceMaps`` (heatmap, paf) that ``find_peaks`` / ``find_connections`` / ``group`` accept directly."""
     import cv2
     import torch
-    if any(float(a) != 0.0 for a in params["rotation_search"]):
-        raise GroupingError("rotation_search other than 0 is not supported by the device post-network stage")
     g = _grouper()
     multiplier = [x * model_params["boxsize"] / image.shape[0] for x in params["scale_search"]]
-    outs, crops = [], []
-    for scale in multiplier:
+    outs, crops, angles = [], [], []
+    for scale, angle in product(multiplier, params["rotation_search"]):  # evaluate.py:89-90
         if scale * image.shape[0] > 2600 or scale * image.shape[1] > 3800:  # evaluate.py:94-96
             scale = min(2600 / image.shape[0], 3800 / image.shape[1])
         image_to_test = cv2.resize(image, (0, 0), fx=scale, fy=scale, interpolation=cv2.INTER_CUBIC)
         padded, _ = pad_right_down_corner(image_to_test, model_params["max_downsample"], model_params["padValue"])
         input_img = np.float32(padded / 255)
+        if angle != 0:  # evaluate.py:108-111; the maps are warped back on the device
+            rotate_matrix = cv2.getRotationMatrix2D((input_img.shape[0] / 2, input_img.shape[1] / 2), angle, 1)
+            input_img = cv2.warpAffine(input_img, rotate_matrix, (0, 0))
         pair = np.concatenate((input_img[None, ...], input_img[:, ::-1, :].copy()[None, ...]), axis=0)
         with torch.no_grad():
             out = model(torch.from_numpy(pair).to(f"cuda:{_device}"))[-1][0]  # last stack, finest scale (:126)
@@ -142,7 +145,9 @@ def predict(image, params, model, model_params, heat_layers=None, paf_layers=Non
             out = out.float()
         outs.append(out[None].contiguous())
         crops.append(image_to_test.shape[:2])
-    heat, paf = g.postnet(outs, crops, image.shape[:2], stride=int(model_params["stride"]), nan_scrub=_variant == "demo")
+        angles.append(float(angle))
+    heat, paf = g.postnet(outs, crops, image.shape[:2], stride=int(model_params["stride"]), nan_scrub=_variant == "demo",
+                          angles=angles)
     return DeviceMaps(heat, False), DeviceMaps(paf, paf.dtype == torch.float32)
 
 

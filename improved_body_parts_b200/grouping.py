@@ -30,7 +30,8 @@ EXPORTS = (
     "spg_assemble", "spg_upload_peaks", "spg_upload_connections", "spg_download_peaks", "spg_download_connections",
     "spg_download_people", "spg_download_status", "spg_launch_count", "spg_stage_kernel", "spg_wire_record_bytes",
     "spg_set_wire_output", "spg_wire_create", "spg_wire_open", "spg_wire_close", "spg_wire_destroy", "spg_wire_signal",
-    "spg_wire_wait", "spg_postnet", "spg_match_assemble", "spg_wire_signal_many", "spg_arm_wire_signal")
+    "spg_wire_wait", "spg_postnet", "spg_match_assemble", "spg_wire_signal_many", "spg_arm_wire_signal",
+    "spg_postnet_rotated")
 
 
 class GroupingError(RuntimeError):
@@ -421,11 +422,14 @@ class Grouper:
     # -- post-network stage ---------------------------------------------------------------------------
     def postnet(self, net_outs, crops, out_hw, *, stride: int = 4, paf_dtype=None, heat_out=None, paf_out=None,
                 paf_chan0: int = 0, heat_chan0: Optional[int] = None, flip_paf_ord=None, flip_heat_ord=None,
-                nan_scrub: bool = False, stream=None):
+                nan_scrub: bool = False, stream=None, angles=None):
         """The scale loop of ``predict()`` after the forward pass (evaluate.py:126-161) on the device.
 
         ``net_outs``: one CUDA tensor ``[N, 2, C, h, w]`` (float32 / float16; image, mirrored image) per scale;
         ``crops``: per scale ``(crop_h, crop_w)`` = ``imageToTest.shape[:2]``; ``out_hw``: the image size.
+        ``angles``: with rotation search, one angle in degrees per entry -- the entries are then the items of
+        ``product(multiplier, rotation_search)`` in that order, each network output computed on the input warped with
+        ``cv2.getRotationMatrix2D((Hp / 2, Wp / 2), angle, 1)`` (evaluate.py:108-111).  All zeros is the same as ``None``.
         Returns ``(heat [N,K,H,W] float32, paf [N,L,H,W])`` -- ``paf`` float32 for a single scale (pass
         ``paf_as_f64=True`` to the grouping calls: the reference's float64 values are exactly these), float64 otherwise.
         """
@@ -466,10 +470,17 @@ class Grouper:
             raise GroupingError("heat_out / paf_out must be contiguous tensors of the requested dtype")
         desc = _PostnetDesc(len(net_outs), scales, int(stride), int(paf_chan0), int(heat_chan0),
                             fp.ctypes.data_as(C.POINTER(C.c_int32)), fh.ctypes.data_as(C.POINTER(C.c_int32)), int(bool(nan_scrub)))
-        rc = self._lib.spg_postnet(self._h, C.byref(desc), C.c_int32(N), C.c_int32(H), C.c_int32(W),
-                                   C.c_void_p(heat_out.data_ptr()), C.c_void_p(paf_out.data_ptr()),
-                                   C.c_int32(F32 if paf_dtype == torch.float32 else F64), self._stream_ptr(stream))
-        self._check(rc, "spg_postnet")
+        out_args = (C.c_int32(N), C.c_int32(H), C.c_int32(W), C.c_void_p(heat_out.data_ptr()), C.c_void_p(paf_out.data_ptr()),
+                    C.c_int32(F32 if paf_dtype == torch.float32 else F64), self._stream_ptr(stream))
+        if angles is None:
+            rc = self._lib.spg_postnet(self._h, C.byref(desc), *out_args)
+            self._check(rc, "spg_postnet")
+        else:
+            ang = np.ascontiguousarray(np.asarray(angles, np.float64).reshape(-1))
+            if ang.shape[0] != len(net_outs):
+                raise GroupingError("one angle per network output expected")
+            rc = self._lib.spg_postnet_rotated(self._h, C.byref(desc), ang.ctypes.data_as(C.POINTER(C.c_double)), *out_args)
+            self._check(rc, "spg_postnet_rotated")
         return heat_out, paf_out
 
     # -- stages -------------------------------------------------------------------------------------

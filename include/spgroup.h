@@ -146,7 +146,7 @@ typedef struct spg_postnet_scale {
     int32_t crop_h, crop_w;         /* imageToTest size: padded size minus pad[2] / pad[3] (evaluate.py:148) */
 } spg_postnet_scale;
 typedef struct spg_postnet_desc {
-    int32_t n_scales;               /* len(multiplier) * len(rotate_angle); rotation is not supported (angle == 0) */
+    int32_t n_scales;               /* items of the loop: len(multiplier) * len(rotate_angle) (spg_postnet: angle 0 only) */
     const spg_postnet_scale *scales;
     int32_t stride;                 /* model_params['stride'] (4) */
     int32_t paf_chan0, heat_chan0;  /* first body-part / keypoint channel of the network output (0 / 30, config.py:101-103) */
@@ -161,6 +161,16 @@ typedef struct spg_postnet_desc {
  * Interpolation follows OpenCV's generic bicubic path (A = -0.75) operation for operation in float32. */
 int spg_postnet(spg_handle *h, const spg_postnet_desc *desc, int32_t n_images, int32_t height, int32_t width,
                 float *heat_out, void *paf_out, int32_t paf_dtype, void *stream);
+/* The same with rotation search (evaluate.py:90-158 with rotation_search != [0]): desc->n_scales counts the items of
+ * product(multiplier, rotate_angle) in the loop's order (scale-major, angle-minor), angle_deg[n_scales] their angles in
+ * degrees.  For an item with angle != 0 the up-sampled maps are warped back over the whole padded image before the crop
+ * -- cv2.warpAffine(map, getRotationMatrix2D((Hp / 2, Wp / 2), -angle, 1), (0, 0)) with Hp = h * stride, Wp = w * stride,
+ * the centre's (rows, cols) order as in the reference -- following OpenCV's fixed-point INTER_LINEAR / BORDER_CONSTANT 0
+ * path bit for bit.  The caller warps the network input with the matching getRotationMatrix2D(..., angle, 1).  Items with
+ * angle 0 take spg_postnet's kernels; all angles 0 is spg_postnet.  Non-finite angles: SPG_E_INVALID.  SPG_F32 body-part
+ * planes need n_scales == 1, as for spg_postnet. */
+int spg_postnet_rotated(spg_handle *h, const spg_postnet_desc *desc, const double *angle_deg, int32_t n_images,
+                        int32_t height, int32_t width, float *heat_out, void *paf_out, int32_t paf_dtype, void *stream);
 
 /* ---- stage entry points (stage-wise parity; each consumes the previous stage's device state) ---- */
 /* find_peaks: evaluate.py:169-203 = util.keypoint_heatmap_nms (utils/util.py:177-183) + util.refine_centroid (:186-211) */

@@ -1,6 +1,6 @@
 #!/usr/bin/env python
 """Small run for compute-sanitizer (memcheck / synccheck): dirty images through every kernel of the library --
-post-network stage (identity, single- and multi-scale, non-identity second resize), persistent, banded and per-item nms / limb_score
+post-network stage (identity, single- and multi-scale, non-identity second resize, rotation search), persistent, banded and per-item nms / limb_score
 (f32, f32-as-f64, f64), fused match+assemble with wire records and the armed signal, the stand-alone match / assemble."""
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
@@ -32,6 +32,8 @@ g2 = Grouper(max_batch=2, max_h=160, max_w=200)
 h1, p1 = g2.postnet([outs[1]], [(90, 120)], (77, 101))
 h3, p3 = g2.postnet(outs, [(48, 64), (96, 128), (192, 256)], (96, 128))
 hi, pi = g2.postnet([outs[1]], [(96, 128)], (96, 128))             # crop == image: the identity kernel
+hr, pr = g2.postnet([outs[1]], [(90, 120)], (77, 101), angles=[22.5])                  # rotation search: one rotated item
+hr3, pr3 = g2.postnet(outs, [(48, 64), (96, 128), (192, 256)], (96, 128), angles=[5.0, 0.0, -90.0])  # rotated / angle-0 launches
 g2.group_device(h3, p3, 96, prm)
 # planes that do not fit shared memory three times: banded nms, body-part planes sampled through L2
 heat3, paf3 = synth.make_batch(7, 2, 150, 260, 8, scale_range=(1.5, 3.0), edge=True)
