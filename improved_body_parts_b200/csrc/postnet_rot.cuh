@@ -6,12 +6,9 @@
 // on the FULL padded up-sampled map (Hp x Wp = h * stride x w * stride), so bilinear taps may land in the padding.
 //
 // Arithmetic of the warp: OpenCV's generic fixed-point path (imgproc/src/imgwarp.cpp, warpAffine + remapBilinear on
-// float32) as restated -- and pinned to cv2 bit for bit -- by tests/rotation_port.py:
-//   the host inverts the matrix in float64 exactly as warpAffine does and passes the destination -> source map m[6];
-//   adelta[x] = rint(m0 x 1024), bdelta[x] = rint(m3 x 1024), X0(y) = rint((m1 y + m2) 1024) + 16,
-//   Y0(y) = rint((m4 y + m5) 1024) + 16 (round half to even); X = (X0 + adelta) >> 5, Y = (Y0 + bdelta) >> 5;
-//   integer tap (Y >> 5, X >> 5), weights the float32 products of 1 - t and t with t = (Y & 31) / 32, (X & 31) / 32;
-//   value p00 w00 + p01 w01 + p10 w10 + p11 w11 in float32, left to right, taps outside [0,Hp) x [0,Wp) reading 0.
+// float32) as restated -- and pinned to cv2 bit for bit -- by tests/rotation_port.py; warp_affine.cuh holds the
+// fixed-point coordinates and weights.  The host inverts the matrix in float64 exactly as warpAffine does and passes
+// the destination -> source map m[6]; taps outside [0,Hp) x [0,Wp) read 0.
 // The resizes and the epilogue are postnet_generic_kernel's operations in the same order; the translation unit is built
 // with -fmad=false and spells out every *_rn operation, so the maps are BIT-IDENTICAL to the port's
 // (tests/test_gpu_postnet_rotation.py).
@@ -30,6 +27,7 @@
 #include <climits>
 
 #include "postnet.cuh"
+#include "warp_affine.cuh"
 
 namespace spg {
 
@@ -81,16 +79,8 @@ __global__ void __launch_bounds__(kPostThreads) postnet_rot_kernel(PostRotArgs r
     const int c_lo = rng[0], FW = rng[1], y_lo = rng[2], FH = rng[3];
     // ---- the warp's fixed-point coordinate tables (warpAffine: AB_BITS = 10, round_delta = 16); the crop starts at
     // the padded map's origin (pad[0] = pad[1] = 0), so crop-grid coordinates are destination coordinates of the warp
-    for (int i = tid; i < FW; i += kPostThreads) {
-        const double x = (double)(c_lo + i);
-        adx[i] = __double2int_rn(__dmul_rn(__dmul_rn(r.m[0], x), 1024.0));
-        bdx[i] = __double2int_rn(__dmul_rn(__dmul_rn(r.m[3], x), 1024.0));
-    }
-    for (int i = tid; i < FH; i += kPostThreads) {
-        const double y = (double)(y_lo + i);
-        x0y[i] = __double2int_rn(__dmul_rn(__dadd_rn(__dmul_rn(r.m[1], y), r.m[2]), 1024.0)) + 16;
-        y0y[i] = __double2int_rn(__dmul_rn(__dadd_rn(__dmul_rn(r.m[4], y), r.m[5]), 1024.0)) + 16;
-    }
+    for (int i = tid; i < FW; i += kPostThreads) warp_col(r.m, c_lo + i, adx[i], bdx[i]);
+    for (int i = tid; i < FH; i += kPostThreads) warp_row(r.m, y_lo + i, x0y[i], y0y[i]);
     __syncthreads();
     if (tid == 0) {
         // source box: X0 + adelta and Y0 + bdelta are sums of a monotone function of x and one of y, so their extremes
@@ -169,11 +159,9 @@ __global__ void __launch_bounds__(kPostThreads) postnet_rot_kernel(PostRotArgs r
         for (int yy = warp; yy < FH; yy += NW) {
             const int X0 = x0y[yy], Y0 = y0y[yy];
             for (int xx = lane; xx < FW; xx += 32) {
-                const int X = (X0 + adx[xx]) >> 5, Y = (Y0 + bdx[xx]) >> 5;
-                const int sx = X >> 5, sy = Y >> 5;
-                const float fx = __fmul_rn((float)(X & 31), 0.03125f), fy = __fmul_rn((float)(Y & 31), 0.03125f);
-                const float gx = __fsub_rn(1.0f, fx), gy = __fsub_rn(1.0f, fy);
-                const float wt[4] = {__fmul_rn(gy, gx), __fmul_rn(gy, fx), __fmul_rn(fy, gx), __fmul_rn(fy, fx)};
+                int sx, sy;
+                float wt[4];
+                warp_tap(X0, Y0, adx[xx], bdx[xx], sx, sy, wt);
                 const bool x0in = sx >= 0 && sx < r.Wp, x1in = sx + 1 >= 0 && sx + 1 < r.Wp;
                 const bool y0in = sy >= 0 && sy < r.Hp, y1in = sy + 1 >= 0 && sy + 1 < r.Hp;
                 const float *p = s2 + (sy - by_lo) * r.cap_bw + (sx - bx_lo);

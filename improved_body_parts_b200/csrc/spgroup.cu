@@ -29,6 +29,7 @@
 #include "nms_peaks_banded.cuh"
 #include "postnet.cuh"
 #include "postnet_rot.cuh"
+#include "prenet.cuh"
 
 using namespace spg;
 
@@ -51,6 +52,8 @@ struct spg_handle {
     unsigned long long armed_value = 0;
     double *heat_acc = nullptr;  // postnet: float64 accumulator of the keypoint maps over the scale loop
     size_t heat_acc_elems = 0;
+    unsigned char *pre_img = nullptr;  // prenet: imageToTest_padded of the current scale, uint8 [Hp][Wp][3]
+    size_t pre_img_bytes = 0;
     cudaStream_t streams[2] = {nullptr, nullptr};
     int64_t launches = 0;
     const char *stage_kernel[5] = {"", "", "", "", ""};  // nms_peaks, limb_score, limb_match, assemble, post-network
@@ -450,6 +453,7 @@ void spg_destroy(spg_handle *h) {
     if (h->in_heat) cudaFree(h->in_heat);
     if (h->in_paf) cudaFree(h->in_paf);
     if (h->heat_acc) cudaFree(h->heat_acc);
+    if (h->pre_img) cudaFree(h->pre_img);
     if (h->done_counter) cudaFree(h->done_counter);
     for (auto &s : h->streams)
         if (s) cudaStreamDestroy(s);
@@ -870,6 +874,86 @@ int spg_postnet_rotated(spg_handle *h, const spg_postnet_desc *d, const double *
             if ((rc = postnet_launch_rotated(h, a, d, t, angle_deg[t], n, H, W, st))) return rc;
             t++;
         }
+    }
+    return SPG_OK;
+}
+
+// ---- pre-network stage -------------------------------------------------------------------------
+namespace {
+
+// cv2.resize(fx = fy = scale)'s dsize (saturate_cast<int>: rint, half to even, in float64) and padRightDownCorner's size
+int prenet_size(spg_handle *h, int32_t height, int32_t width, double scale, int32_t max_downsample, int32_t *crop_h,
+                int32_t *crop_w, int32_t *pad_h, int32_t *pad_w) {
+    if (height < 1 || width < 1 || height > 32767 || width > 32767)
+        return fail(h, SPG_E_INVALID, "image %dx%d outside [1, 32767]", height, width);
+    if (!std::isfinite(scale) || scale <= 0) return fail(h, SPG_E_INVALID, "scale must be finite and > 0");
+    if (max_downsample <= 0) return fail(h, SPG_E_INVALID, "max_downsample must be > 0");
+    const double ch = std::nearbyint((double)height * scale), cw = std::nearbyint((double)width * scale);
+    if (ch < 1 || cw < 1) return fail(h, SPG_E_INVALID, "scale %g resizes a %dx%d image to nothing", scale, height, width);
+    const double ph = std::ceil(ch / max_downsample) * max_downsample, pw = std::ceil(cw / max_downsample) * max_downsample;
+    if (ph > 32767 || pw > 32767)
+        return fail(h, SPG_E_INVALID, "scale %g pads a %dx%d image to %.0fx%.0f, above 32767", scale, height, width, ph, pw);
+    if (crop_h) *crop_h = (int32_t)ch;
+    if (crop_w) *crop_w = (int32_t)cw;
+    if (pad_h) *pad_h = (int32_t)ph;
+    if (pad_w) *pad_w = (int32_t)pw;
+    return SPG_OK;
+}
+
+}  // namespace
+
+int spg_prenet_size(int32_t height, int32_t width, double scale, int32_t max_downsample, int32_t *crop_h, int32_t *crop_w,
+                    int32_t *pad_h, int32_t *pad_w) {
+    return prenet_size(nullptr, height, width, scale, max_downsample, crop_h, crop_w, pad_h, pad_w);
+}
+
+int spg_prenet(spg_handle *h, const unsigned char *image_dev, int64_t row_stride, int32_t height, int32_t width,
+               int32_t channels, double scale, const double *angle_deg, int32_t n_angles, int32_t max_downsample,
+               int32_t pad_value, float *out, int64_t item_stride, void *stream) {
+    if (!h) return SPG_E_INVALID;
+    if (channels != 3) return fail(h, SPG_E_INVALID, "channels = %d: only 3-channel images are supported", channels);
+    if (pad_value < 0 || pad_value > 255) return fail(h, SPG_E_INVALID, "pad_value %d outside [0, 255]", pad_value);
+    int32_t H, W, Hp, Wp;
+    int rc = prenet_size(h, height, width, scale, max_downsample, &H, &W, &Hp, &Wp);
+    if (rc) return rc;
+    if (!image_dev || !out) return fail(h, SPG_E_INVALID, "image_dev/out is NULL");
+    if (row_stride < (int64_t)width * 3) return fail(h, SPG_E_INVALID, "row_stride %lld below width * 3", (long long)row_stride);
+    if (n_angles < 1 || !angle_deg) return fail(h, SPG_E_INVALID, "at least one angle is needed");
+    for (int k = 0; k < n_angles; k++)
+        if (!std::isfinite(angle_deg[k])) return fail(h, SPG_E_INVALID, "angle_deg[%d] is not finite", k);
+    const int64_t item = (int64_t)2 * Hp * Wp * 3;
+    if (n_angles > 1 && item_stride < item) return fail(h, SPG_E_INVALID, "item_stride %lld below 2 * Hp * Wp * 3", (long long)item_stride);
+    DeviceGuard guard(h->device);
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    // the padded image: grown on demand, no other allocation is touched
+    const size_t need = (size_t)Hp * Wp * 3;
+    if (h->pre_img_bytes < need) {
+        if (h->pre_img) cudaFree(h->pre_img);
+        h->pre_img = nullptr; h->pre_img_bytes = 0;
+        SPG_CUDA(h, cudaMalloc(&h->pre_img, need));
+        h->pre_img_bytes = need;
+    }
+    PrenetResizeArgs r{};
+    r.src = image_dev; r.src_row = row_stride; r.h = height; r.w = width; r.H = H; r.W = W; r.Hp = Hp; r.Wp = Wp;
+    r.sx = 1.0 / scale; r.sy = r.sx; r.pad_value = pad_value; r.copy = H == height && W == width; r.dst = h->pre_img;
+    // tile height: the tile's source rows, at most ceil((th - 1) / scale) + 5, fit the shared-memory rows
+    r.tile_h = kPreMaxTH;
+    while (r.tile_h > 1 && std::ceil((r.tile_h - 1) * r.sy) + 5 > kPreRows) r.tile_h /= 2;
+    prenet_resize_kernel<<<dim3((unsigned)((Wp + kPreTW - 1) / kPreTW), (unsigned)((Hp + r.tile_h - 1) / r.tile_h)), kPreThreads, 0, st>>>(r);
+    h->launches++;
+    SPG_CUDA(h, cudaGetLastError());
+    const dim3 grid((unsigned)((Wp + kPreThreads - 1) / kPreThreads), (unsigned)Hp);
+    for (int k = 0; k < n_angles; k++) {
+        PrenetEmitArgs e{};
+        e.img = h->pre_img; e.Hp = Hp; e.Wp = Wp; e.out = out + (int64_t)k * item_stride;
+        if (angle_deg[k] != 0.0) {
+            rotation_inverse_map(angle_deg[k], Hp, Wp, e.m);  // rotate_matrix (evaluate.py:109), inverted as warpAffine does
+            prenet_emit_kernel<true><<<grid, kPreThreads, 0, st>>>(e);
+        } else {
+            prenet_emit_kernel<false><<<grid, kPreThreads, 0, st>>>(e);
+        }
+        h->launches++;
+        SPG_CUDA(h, cudaGetLastError());
     }
     return SPG_OK;
 }

@@ -29,17 +29,21 @@ from .skeleton import COCO_FROM_PART, LIMBS, NUM_PARTS, GroupParams
 _limbs: Tuple[Tuple[int, int], ...] = LIMBS
 _device = 0
 _variant = "evaluate"
+_device_input = False
 _groupers: Dict[int, Grouper] = {}
 CAP_PEAKS, CAP_CANDS, CAP_ROWS = 128, 4096, 128
 MAX_DIM = 32767  # the C ABI's limit; the workspace does not depend on the map size, so ONE handle serves every image size
 
 
 def configure(limbs: Optional[Sequence[Tuple[int, int]]] = None, device: Optional[int] = None,
-              variant: Optional[str] = None) -> None:
-    """Select the limb table (default: the Canonical ``limbs_conn``, config/config.py:94), the CUDA device and the
+              variant: Optional[str] = None, device_input: Optional[bool] = None) -> None:
+    """Select the limb table (default: the Canonical ``limbs_conn``, config/config.py:94), the CUDA device, the
     behavioural variant: ``"evaluate"`` (evaluate.py, the default) or ``"demo"`` (demo_image.py's inlined copy, which
-    differs at :288, :414-415 and :533 -- SURVEY.md 3.2)."""
-    global _limbs, _device, _variant
+    differs at :288, :414-415 and :533 -- SURVEY.md 3.2), and where ``predict`` builds the network input:
+    ``device_input=True`` on the GPU (``Grouper.prenet``), ``False`` (the default) with cv2 on the host as the reference."""
+    global _limbs, _device, _variant, _device_input
+    if device_input is not None:
+        _device_input = bool(device_input)
     if limbs is not None:
         _limbs = tuple((int(a), int(b)) for a, b in limbs)
     if device is not None:
@@ -118,14 +122,20 @@ def pad_right_down_corner(img: np.ndarray, stride: int, pad_value: int) -> Tuple
 def predict(image, params, model, model_params, heat_layers=None, paf_layers=None, input_image_path=None):
     """evaluate.py:83-166 with everything after the forward pass on the device.
 
-    Same arguments as the reference's ``predict``.  The image is scaled and padded exactly as there (cv2, host) and,
-    for an item of ``rotation_search`` with a non-zero angle, rotated with ``cv2.warpAffine`` (:108-111, host); the
-    network runs on the image and its mirror (:116-124), and the flip ensemble, both bicubic resizes, the warp back,
-    the crop and the float64 average over ``product(scale_search, rotation_search)`` (:126-161) happen in
+    Same arguments as the reference's ``predict``.  By default the image is scaled and padded exactly as there (cv2,
+    host) and, for an item of ``rotation_search`` with a non-zero angle, rotated with ``cv2.warpAffine`` (:108-111,
+    host): the network input is bit-identical to the reference's with cv2 as it comes (IPP on).  With
+    ``configure(device_input=True)`` the image goes up once as uint8 (a CUDA uint8 ``[H, W, 3]`` tensor is taken as it
+    is) and ``Grouper.prenet`` builds every item on the GPU: bit-identical to the reference's input with cv2's IPP off
+    (``cv2.ipp.setUseIPP(False)``); with IPP on, cv2's uint8 resize differs by at most 1 in a few percent of the values.
+    The network runs on the image and its mirror (:116-124), and the flip ensemble, both bicubic resizes, the warp
+    back, the crop and the float64 average over ``product(scale_search, rotation_search)`` (:126-161) happen in
     ``spg_postnet`` / ``spg_postnet_rotated`` -- the maps never visit the host.
     Returns two ``DeviceMaps`` (heatmap, paf) that ``find_peaks`` / ``find_connections`` / ``group`` accept directly."""
-    import cv2
     import torch
+    if _device_input:
+        return _predict_device_input(image, params, model, model_params)
+    import cv2
     g = _grouper()
     multiplier = [x * model_params["boxsize"] / image.shape[0] for x in params["scale_search"]]
     outs, crops, angles = [], [], []
@@ -139,16 +149,51 @@ def predict(image, params, model, model_params, heat_layers=None, paf_layers=Non
             rotate_matrix = cv2.getRotationMatrix2D((input_img.shape[0] / 2, input_img.shape[1] / 2), angle, 1)
             input_img = cv2.warpAffine(input_img, rotate_matrix, (0, 0))
         pair = np.concatenate((input_img[None, ...], input_img[:, ::-1, :].copy()[None, ...]), axis=0)
-        with torch.no_grad():
-            out = model(torch.from_numpy(pair).to(f"cuda:{_device}"))[-1][0]  # last stack, finest scale (:126)
-        if out.dtype not in (torch.float32, torch.float16):
-            out = out.float()
-        outs.append(out[None].contiguous())
+        outs.append(_forward(model, torch.from_numpy(pair).to(f"cuda:{_device}")))
         crops.append(image_to_test.shape[:2])
         angles.append(float(angle))
-    heat, paf = g.postnet(outs, crops, image.shape[:2], stride=int(model_params["stride"]), nan_scrub=_variant == "demo",
+    return _postnet(g, outs, crops, image.shape[:2], model_params, angles)
+
+
+def _forward(model, pair):
+    """The forward pass of one item (:116-126): the last stack's finest-scale output, ``[1, 2, C, h, w]``."""
+    import torch
+    with torch.no_grad():
+        out = model(pair)[-1][0]
+    if out.dtype not in (torch.float32, torch.float16):
+        out = out.float()
+    return out[None].contiguous()
+
+
+def _postnet(g: Grouper, outs, crops, image_hw, model_params, angles):
+    import torch
+    heat, paf = g.postnet(outs, crops, image_hw, stride=int(model_params["stride"]), nan_scrub=_variant == "demo",
                           angles=angles)
     return DeviceMaps(heat, False), DeviceMaps(paf, paf.dtype == torch.float32)
+
+
+def _predict_device_input(image, params, model, model_params):
+    """``predict`` with the network input built on the device: one upload, one ``prenet`` per scale."""
+    import torch
+    g = _grouper()
+    dev = torch.device("cuda", _device)
+    if torch.is_tensor(image):
+        img = image.to(dev)
+    else:
+        img = torch.from_numpy(np.ascontiguousarray(image)).to(dev)
+    h, w = int(img.shape[0]), int(img.shape[1])
+    rotation = [float(a) for a in params["rotation_search"]]
+    outs, crops, angles = [], [], []
+    for scale in (x * model_params["boxsize"] / h for x in params["scale_search"]):  # evaluate.py:89-90
+        if scale * h > 2600 or scale * w > 3800:  # evaluate.py:94-96
+            scale = min(2600 / h, 3800 / w)
+        pairs, crop = g.prenet(img, scale, rotation, max_downsample=int(model_params["max_downsample"]),
+                               pad_value=int(model_params["padValue"]))
+        for k, angle in enumerate(rotation):  # product(multiplier, rotate_angle): scale-major, angle-minor
+            outs.append(_forward(model, pairs[k]))
+            crops.append(crop)
+            angles.append(angle)
+    return _postnet(g, outs, crops, (h, w), model_params, angles)
 
 
 def _upload_peaks(g: Grouper, all_peaks) -> None:
@@ -298,13 +343,17 @@ def keypoint_heatmap_nms(heat, kernel: int = 3, thre: float = 0.1):
     return out.to(heat.device)
 
 
-def install(evaluate_module, device_predict: bool = False) -> None:
+def install(evaluate_module, device_predict: bool = False, device_input: bool = False) -> None:
     """Rebind ``find_peaks / find_connections / find_people`` of an imported reference ``evaluate`` module.
 
     ``limbSeq`` is taken from the module (evaluate.py:54) so alternative skeletons keep working.  With
     ``device_predict`` the module's ``predict`` (:83-166) is replaced as well: the network of the module (the global
-    ``posenet`` the reference's own predict uses, :124) feeds the device post-network stage and the maps stay on the GPU."""
-    configure(limbs=getattr(evaluate_module, "limbSeq", _limbs))
+    ``posenet`` the reference's own predict uses, :124) feeds the device post-network stage and the maps stay on the GPU.
+    ``device_input`` (with ``device_predict``) builds the network input on the GPU too -- equal to the reference's
+    with cv2's IPP off, see ``predict``."""
+    if device_input and not device_predict:
+        raise ValueError("device_input needs device_predict")
+    configure(limbs=getattr(evaluate_module, "limbSeq", _limbs), device_input=device_input)
     evaluate_module.find_peaks = find_peaks
     evaluate_module.find_connections = find_connections
     evaluate_module.find_people = find_people

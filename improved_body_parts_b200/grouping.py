@@ -31,7 +31,7 @@ EXPORTS = (
     "spg_download_people", "spg_download_status", "spg_launch_count", "spg_stage_kernel", "spg_wire_record_bytes",
     "spg_set_wire_output", "spg_wire_create", "spg_wire_open", "spg_wire_close", "spg_wire_destroy", "spg_wire_signal",
     "spg_wire_wait", "spg_postnet", "spg_match_assemble", "spg_wire_signal_many", "spg_arm_wire_signal",
-    "spg_postnet_rotated")
+    "spg_postnet_rotated", "spg_prenet_size", "spg_prenet")
 
 
 class GroupingError(RuntimeError):
@@ -101,6 +101,9 @@ def load_library() -> C.CDLL:
         lib.spg_wire_destroy.argtypes = [C.c_int32, C.c_void_p]
         lib.spg_wire_signal.argtypes = [C.c_int32, C.c_void_p, C.c_uint64, C.c_void_p]
         lib.spg_wire_wait.argtypes = [C.c_int32, C.c_void_p, C.c_uint64, C.c_void_p]
+        lib.spg_prenet_size.argtypes = [C.c_int32, C.c_int32, C.c_double, C.c_int32] + [C.POINTER(C.c_int32)] * 4
+        lib.spg_prenet.argtypes = [C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, C.c_int32, C.c_int32, C.c_double,
+                                   C.POINTER(C.c_double), C.c_int32, C.c_int32, C.c_int32, C.c_void_p, C.c_int64, C.c_void_p]
         if lib.spg_abi_version() != ABI_VERSION:
             raise GroupingError("libspgroup.so ABI version mismatch")
         _lib = lib
@@ -253,6 +256,17 @@ def device_bytes_view(ptr: int, nbytes: int, device: int):
     """Zero-copy uint8 torch view of raw device memory."""
     import torch
     return torch.as_tensor(_CudaView(ptr, (int(nbytes),), "|u1"), device=torch.device("cuda", device))
+
+
+def prenet_size(height: int, width: int, scale: float, max_downsample: int = 64):
+    """``spg_prenet_size``: ``((crop_h, crop_w), (Hp, Wp))`` -- ``imageToTest``'s and ``imageToTest_padded``'s sizes
+    for a ``height x width`` image at ``scale`` (evaluate.py:98-100)."""
+    lib = load_library()
+    v = [C.c_int32() for _ in range(4)]
+    rc = lib.spg_prenet_size(int(height), int(width), float(scale), int(max_downsample), *(C.byref(x) for x in v))
+    if rc != 0:
+        raise GroupingError(f"spg_prenet_size failed ({rc}): {(lib.spg_last_error(None) or b'').decode()}")
+    return (v[0].value, v[1].value), (v[2].value, v[3].value)
 
 
 class Grouper:
@@ -418,6 +432,41 @@ class Grouper:
         self._check(rc, "spg_group_host")
         self._last_n = N
         return out
+
+    # -- pre-network stage ----------------------------------------------------------------------------
+    def prenet(self, image, scale: float, angles=(0.0,), *, max_downsample: int = 64, pad_value: int = 128, out=None,
+               stream=None):
+        """What the network sees for every angle of one scale of ``predict()``'s loop (evaluate.py:98-116), built on
+        the device: bicubic resize of the uint8 image, padding to a multiple of ``max_downsample`` with ``pad_value``,
+        ``/ 255``, the rotation by each angle, and the mirrored copy.
+
+        ``image``: CUDA uint8 ``[H, W, 3]`` (BGR, as cv2 reads it) on the handle's device with contiguous pixels; any
+        row stride, so a crop of a larger frame works.  Returns ``(pairs [n_angles, 2, Hp, Wp, 3] float32,
+        (crop_h, crop_w))``: ``pairs[k]`` is the network input of ``angles[k]`` and ``(crop_h, crop_w)`` the
+        ``imageToTest`` size ``postnet`` crops to.  The values equal the reference's with cv2's IPP off, bit for bit;
+        with IPP on (cv2's default) the uint8 resize differs by at most 1 in a few percent of the values."""
+        import torch
+        if not torch.is_tensor(image) or not image.is_cuda or image.device.index != self.device:
+            raise GroupingError(f"image must be a CUDA tensor on cuda:{self.device}")
+        if image.dtype != torch.uint8 or image.dim() != 3 or image.shape[2] != 3:
+            raise GroupingError("image must be a uint8 [H, W, 3] tensor")
+        if image.stride(2) != 1 or image.stride(1) != 3:
+            raise GroupingError("image pixels must be contiguous (pixel stride 3, channel stride 1)")
+        H, W = int(image.shape[0]), int(image.shape[1])
+        (ch, cw), (hp, wp) = prenet_size(H, W, scale, max_downsample)
+        ang = np.ascontiguousarray(np.asarray(angles, np.float64).reshape(-1))
+        if out is None:
+            out = torch.empty((len(ang), 2, hp, wp, 3), dtype=torch.float32, device=torch.device("cuda", self.device))
+        elif out.dtype != torch.float32 or tuple(out.shape) != (len(ang), 2, hp, wp, 3) or not out.is_contiguous() \
+                or not out.is_cuda or out.device.index != self.device:
+            raise GroupingError(f"out must be a contiguous float32 [{len(ang)}, 2, {hp}, {wp}, 3] tensor on cuda:{self.device}")
+        rc = self._lib.spg_prenet(self._h, C.c_void_p(image.data_ptr()), C.c_int64(image.stride(0)), C.c_int32(H),
+                                  C.c_int32(W), C.c_int32(3), C.c_double(float(scale)),
+                                  ang.ctypes.data_as(C.POINTER(C.c_double)), C.c_int32(len(ang)), C.c_int32(int(max_downsample)),
+                                  C.c_int32(int(pad_value)), C.c_void_p(out.data_ptr()), C.c_int64(2 * hp * wp * 3),
+                                  self._stream_ptr(stream))
+        self._check(rc, "spg_prenet")
+        return out, (ch, cw)
 
     # -- post-network stage ---------------------------------------------------------------------------
     def postnet(self, net_outs, crops, out_hw, *, stride: int = 4, paf_dtype=None, heat_out=None, paf_out=None,

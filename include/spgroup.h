@@ -172,6 +172,28 @@ int spg_postnet(spg_handle *h, const spg_postnet_desc *desc, int32_t n_images, i
 int spg_postnet_rotated(spg_handle *h, const spg_postnet_desc *desc, const double *angle_deg, int32_t n_images,
                         int32_t height, int32_t width, float *heat_out, void *paf_out, int32_t paf_dtype, void *stream);
 
+/* ---- pre-network stage: one scale of predict()'s loop before the forward pass, evaluate.py:98-116 ----------- */
+/* Host only, no handle: the sizes spg_prenet produces for a height x width image at `scale` --
+ * crop = imageToTest.shape[:2] = (rint(height * scale), rint(width * scale)) (cv2.resize's dsize, round half to even in
+ * float64; what spg_postnet crops to) and pad = imageToTest_padded.shape[:2] (crop rounded up to multiples of
+ * max_downsample, utils/util.py:44-64).  SPG_E_INVALID for an image outside [1, 32767], a scale that is not finite or
+ * <= 0, max_downsample <= 0, an empty crop or a padded size above 32767; spg_last_error(NULL) gives the reason. */
+int spg_prenet_size(int32_t height, int32_t width, double scale, int32_t max_downsample, int32_t *crop_h, int32_t *crop_w,
+                    int32_t *pad_h, int32_t *pad_w);
+/* The network input of every angle of one scale:
+ *   cv2.resize(image, (0, 0), fx=scale, fy=scale, INTER_CUBIC) -> padRightDownCorner(max_downsample, pad_value) -> / 255
+ *   -> cv2.warpAffine(getRotationMatrix2D((Hp / 2, Wp / 2), angle, 1), (0, 0)) for angle != 0 -> [image, mirrored image]
+ * image_dev: uint8 HWC device image, `channels` must be 3, pixels contiguous, `row_stride` bytes between rows (a crop of
+ * a larger frame works).  out + k * item_stride (elements) receives angle_deg[k]'s item as float32 [2][Hp][Wp][3], the
+ * layout the reference feeds its network.  The resize is OpenCV's 8-bit generic bicubic path without IPP, bit for bit
+ * (cv2 with IPP, its default, differs by at most 1 in a few percent of the uint8 values); the warp is warpAffine's
+ * fixed-point INTER_LINEAR path with border 0, as spg_postnet_rotated's.  Two launches for the first angle, one per
+ * further angle; the padded image lives in handle workspace that grows on demand.  Asynchronous on `stream`.
+ * SPG_E_INVALID for channels != 3, pad_value outside [0, 255], a non-finite angle, and spg_prenet_size's cases. */
+int spg_prenet(spg_handle *h, const unsigned char *image_dev, int64_t row_stride, int32_t height, int32_t width,
+               int32_t channels, double scale, const double *angle_deg, int32_t n_angles, int32_t max_downsample,
+               int32_t pad_value, float *out, int64_t item_stride, void *stream);
+
 /* ---- stage entry points (stage-wise parity; each consumes the previous stage's device state) ---- */
 /* find_peaks: evaluate.py:169-203 = util.keypoint_heatmap_nms (utils/util.py:177-183) + util.refine_centroid (:186-211) */
 int spg_nms_peaks(spg_handle *h, const float *heat_dev, int64_t image_stride, int64_t chan_stride,

@@ -1,6 +1,7 @@
 #!/usr/bin/env python
 """Small run for compute-sanitizer (memcheck / synccheck): dirty images through every kernel of the library --
-post-network stage (identity, single- and multi-scale, non-identity second resize, rotation search), persistent, banded and per-item nms / limb_score
+pre-network stage (strided image, rotated and not), post-network stage (identity, single- and multi-scale, non-identity
+second resize, rotation search), persistent, banded and per-item nms / limb_score
 (f32, f32-as-f64, f64), fused match+assemble with wire records and the armed signal, the stand-alone match / assemble."""
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
@@ -35,10 +36,16 @@ hi, pi = g2.postnet([outs[1]], [(96, 128)], (96, 128))             # crop == ima
 hr, pr = g2.postnet([outs[1]], [(90, 120)], (77, 101), angles=[22.5])                  # rotation search: one rotated item
 hr3, pr3 = g2.postnet(outs, [(48, 64), (96, 128), (192, 256)], (96, 128), angles=[5.0, 0.0, -90.0])  # rotated / angle-0 launches
 g2.group_device(h3, p3, 96, prm)
+# pre-network stage: a strided crop of a larger frame, angle 0 and rotated items, a copy (dsize == ssize) and a down-scale
+frame = torch.from_numpy(np.random.default_rng(3).integers(0, 256, (130, 190, 3), dtype=np.uint8)).to(dev)
+crop = frame[7:127, 13:173]
+pairs, _ = g2.prenet(crop, 1.37, [0.0, -5.0, 22.5])
+pairs1, _ = g2.prenet(crop, 1.0, [0.0], max_downsample=8, pad_value=0)
+pairs2, _ = g2.prenet(crop, 0.21, [90.0])
 # planes that do not fit shared memory three times: banded nms, body-part planes sampled through L2
 heat3, paf3 = synth.make_batch(7, 2, 150, 260, 8, scale_range=(1.5, 3.0), edge=True)
 g3 = Grouper(max_batch=2, max_h=150, max_w=260)
 g3.group_device(torch.from_numpy(heat3).to(dev), torch.from_numpy(paf3).to(dev), 150, prm)
 k3 = g3.stage_kernels()
 torch.cuda.synchronize()
-print("persons", r.n_persons.tolist(), "status", r.status.tolist(), "kernels", k1, g.stage_kernels(), "postnet", tuple(h1.shape), tuple(p3.shape), tuple(hi.shape), "large planes", k3)
+print("persons", r.n_persons.tolist(), "status", r.status.tolist(), "kernels", k1, g.stage_kernels(), "postnet", tuple(h1.shape), tuple(p3.shape), tuple(hi.shape), "large planes", k3, "prenet", tuple(pairs.shape))
